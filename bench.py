@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — images/sec of one compression-aware training step (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--workload NAME] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload NAME] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch of synthetic input: teacher forward (eval mode),
@@ -18,6 +18,8 @@ gradient all-reduce (N > 1), fused optimizer.  Nothing is skipped inside the tim
   cpu_baseline  : the oracle step (oracle/step_oracle.py: un-fused PyTorch-CPU fp32, all host cores)
                   on a bounded sample of the same workload (TF 1.x cannot run in this image).
 `--impl reference` times that CPU path alone (rank 0 only) and prints the same line.
+`--dump-outputs DIR` writes what the last timed step handed its caller (see dump_outputs); inputs and initial weights are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -144,6 +146,27 @@ def peaks():
         d = json.load(open(p))
         return d['hbm_gbs'], d['bf16_tflops'], d.get('bf16_tflops_sustained', d['bf16_tflops']), 'measured'
     return 6650.0, 1590.0, 1400.0, 'fallback'
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE = 1 << 16
+
+
+def dump_outputs(out_dir, losses, state):
+    """<out_dir>/loss.<term>.npy for every loss term of the step and <out_dir>/var.<variable>.npy for every model variable
+    after it ('/' -> '.', ':' -> '_'), float32.  A variable larger than the per-variable share of DUMP_LIMIT_BYTES (at
+    most DUMP_SAMPLE elements) is written as the 1-D sample of its flattened entries at sorted indices drawn by
+    np.random.default_rng(0): the same entries in every run of the same workload."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {'loss.' + k: np.asarray(v, np.float32) for k, v in losses.items()}
+    per_var = max(1, min(DUMP_SAMPLE, (DUMP_LIMIT_BYTES // 4 - len(arrays)) // max(len(state), 1)))
+    for name, v in state.items():
+        a = np.asarray(v, np.float32)
+        if a.size > per_var:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, per_var, replace=False))]
+        arrays['var.' + name.replace('/', '.').replace(':', '_')] = a
+    for n, a in arrays.items():
+        np.save(os.path.join(out_dir, n + '.npy'), a)
 
 
 def build_learner(workload, world, batch_override=None):
@@ -350,7 +373,13 @@ def main():
     ap.add_argument('--cpu-batch', type=int, default=None)
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-graph', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the losses of the last timed step and the model variables after it to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs applies to --impl b200')
     quiet_stdout()
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
@@ -433,6 +462,8 @@ def main():
         dist.all_reduce(ms2, op=dist.ReduceOp.MAX)
     e2e_ms = float(ms2.item())
     sampler.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, losses, ex.store.state_dict())
     # ---- instrumented eager step: per-group device time for the roofline
     hbm_peak, tf_peak, tf_sust, peak_kind = peaks()
     prof = ex.profile_step(lr, allreduce)

@@ -215,6 +215,29 @@ def test_bench_reference_arm_prints_one_contract_line():
     assert d['e2e']['h2d_bytes_per_step'] == 0 and d['e2e']['d2h_bytes_per_step'] == 0
 
 
+def test_bench_dump_outputs_is_reproducible_and_bounded(tmp_path):
+    """bench.dump_outputs: float32 .npy per loss term and per variable, large variables sampled at the same indices in
+    every run, the whole dump within DUMP_LIMIT_BYTES even when the model has many large variables."""
+    import bench
+    rng = np.random.default_rng(5)
+    losses = {'loss': F32(2.5), 'ce': F32(2.25)}
+    state = {'model/conv/kernel:0': rng.standard_normal((3, 3, 64, 128)).astype(F32),
+             'model/bn/beta:0': rng.standard_normal(64).astype(F32)}
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), losses, state)
+    names = sorted(os.listdir(str(tmp_path / 'a')))
+    assert names == ['loss.ce.npy', 'loss.loss.npy', 'var.model.bn.beta_0.npy', 'var.model.conv.kernel_0.npy']
+    for n in names:
+        a, b = np.load(str(tmp_path / 'a' / n)), np.load(str(tmp_path / 'b' / n))
+        assert a.dtype == F32 and np.array_equal(a, b), n
+    assert np.array_equal(np.load(str(tmp_path / 'a' / 'var.model.bn.beta_0.npy')), state['model/bn/beta:0'])
+    k = np.load(str(tmp_path / 'a' / 'var.model.conv.kernel_0.npy'))
+    assert k.shape == (bench.DUMP_SAMPLE,) and np.isin(k, state['model/conv/kernel:0']).all()
+    big = {'v%d' % i: np.zeros(bench.DUMP_SAMPLE + 1, F32) for i in range(300)}
+    bench.dump_outputs(str(tmp_path / 'c'), losses, big)
+    assert sum(os.path.getsize(str(p)) for p in (tmp_path / 'c').iterdir()) <= bench.DUMP_LIMIT_BYTES + 128 * 302
+
+
 def test_run_scripts_parse_flags_and_map_value_errors_to_exit_status_1(capsys):
     """nets/*_run.py: every learner's flags are known before parsing; a bad execution mode or learner name is a
     ValueError -> exit status 1 (nets/resnet_at_cifar10_run.py:62-66), not a traceback to the shell."""

@@ -156,9 +156,9 @@ def test_full_prec_learner_and_checkpoint_roundtrip(tmp_path):
     assert np.isfinite(lrn.evaluate())
 
 
-def test_uniform_learner_trains_and_evaluates():
+def test_uniform_learner_trains_and_evaluates(tmp_path):
     lrn = make('uniform', uql_weight_bits=8, uql_use_buckets=True, enbl_dst=True, summ_step=5, save_step=10 ** 9,
-               uql_save_quant_model_path='/tmp/pf_uql_test/model.ckpt')
+               uql_save_quant_model_path=str(tmp_path / 'uql' / 'model.ckpt'))
     lrn.train(nb_iters=6)            # includes the CUDA-graph-free eager loop, logging, final save + evaluate
     r = lrn.sess_train.fetch_losses()
     assert np.isfinite(r['loss']) and lrn.sess_train.step_count == 6
