@@ -227,6 +227,42 @@ int pf_nuq_cluster_grad(const pf_uq_seg* gsegs_dev, int n_seg, const pf_work* wo
                         const float* scales_dev, float* partial_ws_dev, float* grad_base_dev,
                         const int64_t* cluster_off_dev, void* stream);
 
+/* a11b Bucketed codebooks (--nuql_use_buckets): NonUniformQuantization.__bucket_quantize /
+ *     __build_bucket_norm_quant_point / __quantile_init(axis=0) — learners/nonuniform_quantization/utils.py:196-243,
+ *     309-366.  One codebook per bucket (bucket of flat element i = i % ncols, the layout of pf_uq_seg with
+ *     split / channel buckets) and the per-bucket scales of pf_uq_weight_minmax + pf_uq_weight_scales.  The
+ *     codebooks of tensor `seg` are the [2^bits', ncols] row-major `clusters` variable at
+ *     clusters_base_dev + cluster_off_dev[seg] (bits' >= bits): centroid j of bucket b at + j*ncols + b.
+ *
+ *     Quantize: work = kind-1 column tiles (rows [start, start+count) x columns [c0, c0+ncol_tile) of the
+ *     [padded/ncols, ncols] view) with (2^bits + 3) * ncol_tile <= PF_NUQ_BUCKET_TILE_FLOATS + 3 * ncol_tile and
+ *     ncol_tile <= PF_NUQ_BUCKET_MAX_TILE.  Only elements with flat index < numel are written; idx_out as in
+ *     pf_nuq_weight_quant. */
+#define PF_NUQ_BUCKET_TILE_FLOATS 8192
+#define PF_NUQ_BUCKET_MAX_TILE 1024
+#define PF_NUQ_BUCKET_MAX_ROWS 16384
+#define PF_NUQ_BUCKET_GRAD_TILE 32
+int pf_nuq_bucket_weight_quant(const pf_uq_seg* segs_dev, const pf_work* work_dev, int n_work,
+                               const float* scales_dev, int n_buckets, const float* clusters_base_dev,
+                               const int64_t* cluster_off_dev, uint8_t* idx_out_dev, const int64_t* idx_base_dev,
+                               void* stream);
+/* Quantile init, one CTA per bucket slot (n_buckets = the scales' slot count): centroid j of bucket b =
+ *     x_n at descending rank ranks_dev[seg*256 + j] of the bucket's padded/ncols rows (padding rows = copies of the
+ *     last element, counted as the reference counts them), x_n = (w-beta)/alpha in fp32.  Writes rows 0..2^bits-1 of
+ *     each codebook.  max_rows = the tallest bucket, at most PF_NUQ_BUCKET_MAX_ROWS (sorted in shared memory). */
+int pf_nuq_bucket_quantile_init(const pf_uq_seg* segs_dev, int n_seg, const float* scales_dev, int n_buckets,
+                                const int32_t* ranks_dev, int max_rows, float* clusters_base_dev,
+                                const int64_t* cluster_off_dev, void* stream);
+/* Codebook gradient, dL/dc[j,b] = alpha_b * sum_{i < numel, i % ncols = b, idx_i = j} g_i.  work: kind-1 tiles of at
+ *     most PF_NUQ_BUCKET_GRAD_TILE columns x a row range; tiles_dev[t]: seg, c0, ncol_tile of column tile t and, in
+ *     start/count, the contiguous range of its work items; partial_ws_dev: n_work * kmax * PF_NUQ_BUCKET_GRAD_TILE
+ *     floats (kmax >= every 2^bits).  Deterministic (fixed-order two-stage reduction); writes only rows 0..2^bits-1
+ *     of the codebooks in grad_base_dev (layout of clusters_base_dev). */
+int pf_nuq_bucket_cluster_grad(const pf_uq_seg* gsegs_dev, const pf_work* work_dev, int n_work,
+                               const pf_work* tiles_dev, int n_tiles, int kmax, const uint8_t* idx_dev,
+                               const int64_t* idx_base_dev, const float* scales_dev, float* partial_ws_dev,
+                               float* grad_base_dev, const int64_t* cluster_off_dev, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * a4  Convolution / dense layers, exact-fp32 CUDA-core path (pf_conv.cu).
  *     Replaces tf.nn.conv2d / tf.matmul re-created on the quantized weight

@@ -272,7 +272,14 @@ class Executor:
                 # live in the parameter store), else a private table of the quantizer
                 cvars = [op.vars.get('clusters') for op in self.wq_ops]
                 self.train_clusters = bool(wq.get('train_clusters', False)) and self.train
-                if all(c is not None for c in cvars):
+                if wq.get('use_buckets', False):
+                    # per-bucket codebooks: always the [k, ncols] `clusters` variables of the graph edit.  They are
+                    # consumed through QW like every codebook (the integer-level conv operands are uniform-only)
+                    self.wq = ops.CodebookWeightQuantizer(srcs, dsts, wq['bits'], keep_index=self.train_clusters,
+                                                          cluster_views=[st.view(c) for c in cvars], cluster_base=st.P,
+                                                          use_buckets=True, bucket_type=wq['bucket_type'],
+                                                          bucket_size=wq['bucket_size'])
+                elif all(c is not None for c in cvars):
                     self.wq = ops.CodebookWeightQuantizer(srcs, dsts, wq['bits'], keep_index=self.train_clusters,
                                                           cluster_views=[st.view(c) for c in cvars], cluster_base=st.P)
                 else:

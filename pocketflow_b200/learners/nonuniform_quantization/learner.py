@@ -131,7 +131,17 @@ class NonUniformQuantLearner(AbstractLearner):
             self.feed(ex, self.eval_iterator())
             ex.forward_eval_loss()
             out.append(ex.fetch_losses()['loss'])
+        if FLAGS.nuql_use_buckets:
+            self.__show_bucket_storage(self.bucket_storage)
         return float(np.mean(out))
+
+    def __show_bucket_storage(self, bucket_storage):
+        """learner.py:470-476: the per-bucket alpha / beta against the quantized weights' own bits"""
+        bits = FLAGS.nuql_weight_bits if not FLAGS.nuql_enbl_rl_agent else FLAGS.nuql_equivalent_bits
+        weight_storage = sum(self.statistics['num_weights']) * bits
+        print('bucket storage: %d bit / %.3f kb | weight storage: %d bit / %.3f kb | ratio: %.3f'
+              % (bucket_storage, bucket_storage / (8. * 1024.), weight_storage, weight_storage / (8. * 1024.),
+                 bucket_storage * 1. / weight_storage))
 
     # ------------------------------------------------------------------ what the RL bit search drives
     def rl_restore(self):
@@ -203,6 +213,7 @@ class NonUniformQuantLearner(AbstractLearner):
                 self.optimal_w_bit_list, self.optimal_a_bit_list = w_bits, a_bits
                 nq.insert_quant_op_for_weights({op.name: b for op, b in zip(matmul_ops, w_bits)})
                 nq.insert_quant_op_for_activations({op.name: b for op, b in zip(act_ops, a_bits)})
+                self.bucket_storage = nq.bucket_storage
                 # "Strictly speaking, clusters should be not included for regularization" (learner.py:219-220): they are
                 loss, metrics = self.calc_loss(labels, logits, self.trainable_vars)
                 if FLAGS.enbl_dst:

@@ -3,6 +3,7 @@
 quantizer (pf_nuq_weight_quant), activations through the UNIFORM quantizer (utils.py:58-85)."""
 import numpy as np
 
+from ...ops import nuq_bucket_layout
 from ..uniform_quantization.utils import prefix_filter
 
 
@@ -28,9 +29,11 @@ class NonUniformQuantization:
             raise ValueError("Unrecognized bucket type, must be 'weight' or 'channel'.")
         if self.init_style not in ('quantile', 'uniform'):
             raise ValueError("Unrecognized Initialization Mode.")
-        if self.use_buckets:
-            raise NotImplementedError('bucketed codebooks are not built yet (per-layer codebooks only); the '
-                                      'reference\'s bucketed uniform init is itself broken (SURVEY A.6-6)')
+        if self.use_buckets and self.init_style == 'uniform':
+            # __bucket_quantize calls __uniform_init(x_normalized, k) (utils.py:225) against its signature
+            # __uniform_init(nb_clusters, bucket_num=0) (:368): the reference cannot run this combination
+            raise ValueError('--nuql_init_style uniform with --nuql_use_buckets is broken in the reference '
+                             '(__uniform_init is called with the wrong arguments, SURVEY A.6-6); use quantile')
         self.support_act_types = ['Relu', 'Relu6', 'Crelu', 'Elu', 'Selu', 'Softplus', 'Softsign', 'Sigmoid', 'Tanh']
         self.support_mul_types = ['Conv2D', 'MatMul', 'DepthwiseConv2dNative']
 
@@ -60,7 +63,15 @@ class NonUniformQuantization:
             bits = int(w_bit_dict[op.name])
             self.quantized_matmul_ops.append(op)
             self.weight_bits.append(bits)
-            if op.type != 'DepthwiseConv2dNative' and bits <= 8:
+            if self.use_buckets:
+                # __bucket_quantize: a [k, bucket_num] `clusters` variable under <prefix>/nonuniform_bucket_quantize
+                # (utils.py:209, :324) for EVERY quantized op, depthwise included; bucket_storage as :487-494
+                ncols, _, _ = nuq_bucket_layout(op.vars['kernel'].shape, self.bucket_type, self.bucket_size)
+                name = g.scope_prefix() + prefix_filter(op.name) + '/nonuniform_bucket_quantize/clusters'
+                op.vars['clusters'] = g.get_variable(name, (2 ** max(bits, self.codebook_bits_cap or 0), ncols),
+                                                     lambda rng, shape: np.zeros(shape, np.float32), trainable=True)
+                self.bucket_storage += ncols * 32 * 2
+            elif op.type != 'DepthwiseConv2dNative' and bits <= 8:
                 name = g.scope_prefix() + prefix_filter(op.name) + '/nonuniform_quantize/clusters'
                 op.vars['clusters'] = g.get_variable(name, (2 ** max(bits, self.codebook_bits_cap or 0),), lambda rng, shape: np.zeros(shape, np.float32),
                                                      trainable=True)
@@ -75,8 +86,11 @@ class NonUniformQuantization:
     def weight_quant_spec(self):
         if not self.quantized_matmul_ops:
             return None
-        return dict(kind='nonuniform', ops=self.quantized_matmul_ops, bits=self.weight_bits,
+        spec = dict(kind='nonuniform', ops=self.quantized_matmul_ops, bits=self.weight_bits,
                     init_style=self.init_style, train_clusters=False)
+        if self.use_buckets:
+            spec.update(use_buckets=True, bucket_type=self.bucket_type, bucket_size=self.bucket_size)
+        return spec
 
     def act_quant_spec(self):
         if not self.quantized_activation_ops:

@@ -37,6 +37,10 @@ SIGNATURES = {
     'pf_nuq_weight_quant': (c_i32, [c_vp, c_vp, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_vp]),
     'pf_nuq_weight_quant_ex': (c_i32, [c_vp, c_vp, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp]),
     'pf_nuq_cluster_grad': (c_i32, [c_vp, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    'pf_nuq_bucket_weight_quant': (c_i32, [c_vp, c_vp, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    'pf_nuq_bucket_quantile_init': (c_i32, [c_vp, c_i32, c_vp, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp]),
+    'pf_nuq_bucket_cluster_grad': (c_i32, [c_vp, c_vp, c_i32, c_vp, c_i32, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                                           c_vp]),
     'pf_im2col': (c_i32, [c_vp, c_vp, c_i32, c_vp, c_vp]),
     'pf_s2d_planes': (c_i32, [c_vp] + [c_i32] * 9 + [c_vp, c_vp, c_vp]),
     'pf_preprocess_images': (c_i32, [c_vp, c_vp, c_i32, c_i32, c_i32, c_f32, c_f32, c_f32, c_vp, c_vp]),

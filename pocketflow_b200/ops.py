@@ -73,6 +73,55 @@ def minmax_works(segs):
     return np.array(rows, dtype=WORK) if rows else np.zeros(0, dtype=WORK)
 
 
+NUQ_BUCKET_TILE_FLOATS = 8192   # PF_NUQ_BUCKET_TILE_FLOATS: codebook slice of one quantize work item
+NUQ_BUCKET_MAX_TILE = 1024      # PF_NUQ_BUCKET_MAX_TILE
+NUQ_BUCKET_MAX_ROWS = 16384     # PF_NUQ_BUCKET_MAX_ROWS: tallest bucket the quantile init sorts in shared memory
+NUQ_BUCKET_GRAD_TILE = 32       # PF_NUQ_BUCKET_GRAD_TILE
+
+
+def nuq_bucket_layout(shape, bucket_type, bucket_size):
+    """(ncols, padded, rows) of a weight under bucketed codebooks: the [rows, ncols] view of __split_bucket /
+    __channel_bucket (learners/nonuniform_quantization/utils.py:435-476).  A ValueError for buckets taller than the
+    quantile init can sort (only reachable with a large --nuql_bucket_size, or channel buckets of a huge kernel)."""
+    ncols, padded = uq_bucket_layout(shape, True, bucket_type, bucket_size)
+    rows = padded // ncols
+    if rows > NUQ_BUCKET_MAX_ROWS:
+        raise ValueError('bucketed codebooks: a bucket of %d rows (weight %s, %s buckets) exceeds the %d rows the '
+                         'quantile init supports' % (rows, tuple(shape), bucket_type, NUQ_BUCKET_MAX_ROWS))
+    return ncols, padded, rows
+
+
+def nuq_bucket_quant_works(segs):
+    """kind-1 column tiles of pf_nuq_bucket_weight_quant: a tile's codebook slice (2^bits x tile floats) fits
+    NUQ_BUCKET_TILE_FLOATS; about 16K elements per work item."""
+    rows = []
+    for s, seg in enumerate(segs):
+        ncols, padded, nc = int(seg['ncols']), int(seg['padded']), 1 << int(seg['bits'])
+        tile = min(ncols, NUQ_BUCKET_MAX_TILE, max(32, NUQ_BUCKET_TILE_FLOATS // nc))
+        nrows = padded // ncols
+        rows_per = max(1, 16384 // tile)
+        for c0 in range(0, ncols, tile):
+            for r0 in range(0, nrows, rows_per):
+                rows.append((s, 1, r0, min(rows_per, nrows - r0), c0, min(tile, ncols - c0), 0))
+    return np.array(rows, dtype=WORK) if rows else np.zeros(0, dtype=WORK)
+
+
+def nuq_bucket_grad_works(segs, rows_per=256):
+    """(work, tiles) of pf_nuq_bucket_cluster_grad: NUQ_BUCKET_GRAD_TILE columns x rows_per rows per work item; tile t
+    lists its contiguous work items in start/count."""
+    work, tiles = [], []
+    for s, seg in enumerate(segs):
+        ncols, padded = int(seg['ncols']), int(seg['padded'])
+        nrows = padded // ncols
+        for c0 in range(0, ncols, NUQ_BUCKET_GRAD_TILE):
+            tc = min(NUQ_BUCKET_GRAD_TILE, ncols - c0)
+            first = len(work)
+            for r0 in range(0, nrows, rows_per):
+                work.append((s, 1, r0, min(rows_per, nrows - r0), c0, tc, 0))
+            tiles.append((s, 1, first, len(work) - first, c0, tc, 0))
+    return np.array(work, dtype=WORK), np.array(tiles, dtype=WORK)
+
+
 def percentile_rank_desc(n, q):
     """Index into the descending sort gathered by tf.contrib.distributions.percentile
     (interpolation='nearest'): clip(int32(rint((n-1)*(1-q/100))), 0, n-1) in float64."""
@@ -386,25 +435,42 @@ class CodebookWeightQuantizer:
 
     The codebooks are either a private [tensors, 256] table (`clusters`), or — `cluster_views` — 1-D views of ONE flat
     buffer `cluster_base` that the caller owns: the reference's trainable `clusters` variables (utils.py:297), which then
-    sit among the model's parameters (optimizer, weight decay, checkpoints, broadcast all apply to them)."""
+    sit among the model's parameters (optimizer, weight decay, checkpoints, broadcast all apply to them).
 
-    def __init__(self, srcs, dsts, bits, keep_index=False, cluster_views=None, cluster_base=None):
+    use_buckets (NonUniformQuantization.__bucket_quantize, utils.py:196-243): one codebook per 'split' / 'channel'
+    bucket, ranges per bucket through the bucketed UniformWeightQuantizer.  The codebooks of a tensor are then a
+    [2^bits, ncols] row-major table — a view of cluster_base (the reference's [k, bucket_num] `clusters` variable), or
+    a private buffer when no views are given."""
+
+    def __init__(self, srcs, dsts, bits, keep_index=False, cluster_views=None, cluster_base=None, use_buckets=False,
+                 bucket_type='split', bucket_size=256):
         self.L = _lib.load()
         _check_f32(*srcs)
         _check_f32(*dsts)
-        self.uq = UniformWeightQuantizer(srcs, dsts, bits)       # per-layer ranges + tables
+        self.use_buckets = bool(use_buckets)
+        if self.use_buckets:
+            for s in srcs:
+                nuq_bucket_layout(tuple(s.shape), bucket_type, bucket_size)     # bucket height, before any launch
+        # per-layer or per-bucket ranges + tables
+        self.uq = UniformWeightQuantizer(srcs, dsts, bits, self.use_buckets, bucket_type, bucket_size)
         if any(b > 8 for b in self.uq.bits):
             raise ValueError('codebook bit-widths must be <= 8')
         self.srcs, self.dsts = list(srcs), list(dsts)
         self.device = self.uq.device
+        self.ncols = [int(s['ncols']) for s in self.uq.segs]
         self.cluster_views, self.cluster_base, self.cluster_off = None, None, None
+        if cluster_views is None and self.use_buckets:
+            sizes = [(1 << b) * nc for b, nc in zip(self.uq.bits, self.ncols)]
+            offs = np.concatenate([[0], np.cumsum([(n + 3) // 4 * 4 for n in sizes])]).astype(np.int64)
+            cluster_base = torch.zeros(max(int(offs[-1]), 4), dtype=torch.float32, device=self.device)
+            cluster_views = [cluster_base[o:o + n].view(-1, nc) for o, n, nc in zip(offs, sizes, self.ncols)]
         if cluster_views is not None:
             _check_f32(cluster_base, *cluster_views)
             offs = []
-            for v, b in zip(cluster_views, self.uq.bits):
+            for v, b, nc in zip(cluster_views, self.uq.bits, self.ncols):
                 off = (v.data_ptr() - cluster_base.data_ptr()) // 4
-                if v.numel() < (1 << b) or off < 0 or off + v.numel() > cluster_base.numel():
-                    raise ValueError('codebook views must hold at least 2^bits floats inside cluster_base')
+                if v.numel() < (1 << b) * nc or v.numel() % nc or off < 0 or off + v.numel() > cluster_base.numel():
+                    raise ValueError('codebook views must hold at least 2^bits x buckets floats inside cluster_base')
                 offs.append(off)
             self.cluster_views, self.cluster_base = list(cluster_views), cluster_base
             self.cluster_off = torch.tensor(offs, dtype=torch.int64, device=self.device)
@@ -421,6 +487,24 @@ class CodebookWeightQuantizer:
             self.idx_base = torch.tensor(offs, dtype=torch.int64, device=self.device)
             self.idx_offsets = offs
         self._grad_tables = None
+        if self.use_buckets:
+            self._bucket_tables()
+
+    def _bucket_tables(self):
+        """Work tables of the bucketed kernels for the current bit-widths."""
+        segs = self.uq.segs
+        self.work_bq = nuq_bucket_quant_works(segs)
+        self.work_bg, self.tiles_bg = nuq_bucket_grad_works(segs)
+        self.work_bq_dev = _upload(self.work_bq, self.device)
+        self.work_bg_dev = _upload(self.work_bg, self.device)
+        self.tiles_bg_dev = _upload(self.tiles_bg, self.device)
+        self.kmax = max([1 << b for b in self.uq.bits] or [1])
+        self.max_rows = max([int(s['padded']) // int(s['ncols']) for s in segs] or [1])
+        ranks = np.zeros((max(len(segs), 1), 256), np.int32)
+        for i, s in enumerate(segs):
+            k, rows = 1 << int(s['bits']), int(s['padded']) // int(s['ncols'])
+            ranks[i, :k] = [percentile_rank_desc(rows, (j + 1) * 100 / (k + 1)) for j in range(k)]
+        self.ranks_dev = _upload(ranks, self.device)
 
     def quantile_values(self):
         """clusters_j = percentile(x_n, (j+1)*100/(k+1)) (utils.py:349-366), [tensors][k] as numpy.  x -> x_n is
@@ -444,17 +528,31 @@ class CodebookWeightQuantizer:
         return out
 
     def set_bits(self, bits):
-        """New bit-widths (the RL bit search): a codebook keeps its place and uses its first 2^bits entries; call
-        quantile_init() afterwards."""
+        """New bit-widths (the RL bit search): a codebook keeps its place and uses its first 2^bits entries (per-bucket
+        codebooks: the first 2^bits rows of the [k, ncols] table); call quantile_init() afterwards."""
         bits = [int(b) for b in (bits if hasattr(bits, '__len__') else [bits] * len(self.srcs))]
         if any(b < 1 or b > 8 for b in bits):
             raise ValueError('codebook bit-widths must be in [1, 8]')
-        if self.cluster_views is not None and any(v.numel() < (1 << b) for v, b in zip(self.cluster_views, bits)):
+        if self.cluster_views is not None and any(v.numel() < (1 << b) * nc
+                                                  for v, b, nc in zip(self.cluster_views, bits, self.ncols)):
             raise ValueError('a codebook variable is smaller than 2^bits')
         self.uq.set_bits(bits)
         self._grad_tables = None
+        if self.use_buckets:
+            self._bucket_tables()
 
     def quantile_init(self):
+        if self.use_buckets:
+            # __quantile_init(axis=0) per bucket, on the device, straight into the codebook tables
+            self.uq.minmax()
+            for v, b, nc in zip(self.cluster_views, self.uq.bits, self.ncols):
+                if v.numel() > (1 << b) * nc:
+                    v.zero_()                               # rows past 2^bits stay 0 (no weight-decay term)
+            _lib.check(self.L.pf_nuq_bucket_quantile_init(_p(self.uq.segs_dev), len(self.srcs), _p(self.uq.scales),
+                                                          self.uq.n_buckets, _p(self.ranks_dev), self.max_rows,
+                                                          _p(self.cluster_base), _p(self.cluster_off), _stream()),
+                       'pf_nuq_bucket_quantile_init')
+            return
         vals = self.quantile_values()
         if self.cluster_views is not None:
             for v, c in zip(self.cluster_views, vals):
@@ -469,7 +567,12 @@ class CodebookWeightQuantizer:
     def forward(self):
         self.uq.minmax()
         idx_base = _p(self.idx_base) if self.idx is not None else None
-        if self.cluster_views is not None:
+        if self.use_buckets:
+            _lib.check(self.L.pf_nuq_bucket_weight_quant(_p(self.uq.segs_dev), _p(self.work_bq_dev), len(self.work_bq),
+                                                         _p(self.uq.scales), self.uq.n_buckets, _p(self.cluster_base),
+                                                         _p(self.cluster_off), _p(self.idx), idx_base, _stream()),
+                       'pf_nuq_bucket_weight_quant')
+        elif self.cluster_views is not None:
             _lib.check(self.L.pf_nuq_weight_quant_ex(_p(self.uq.segs_dev), _p(self.uq.work_q_dev), len(self.uq.work_q),
                                                      _p(self.uq.scales), self.uq.n_buckets, _p(self.cluster_base),
                                                      _p(self.cluster_off), _p(self.idx), idx_base, _stream()),
@@ -487,6 +590,22 @@ class CodebookWeightQuantizer:
             raise ValueError('cluster_grad needs keep_index=True and cluster_views')
         _check_f32(grad_base, *grads)
         ptrs = [g.data_ptr() for g in grads]
+        if self.use_buckets:
+            # dL/dc[j, b] = alpha_b * sum_{idx = j} g over the bucket's rows (padding rows excluded)
+            if self._grad_tables is None or self._grad_tables[0] != ptrs:
+                gs = self.uq.segs.copy()
+                gs['src'] = ptrs
+                gs['dst'] = ptrs
+                self._grad_tables = (ptrs, _upload(gs, self.device),
+                                     torch.empty(max(len(self.work_bg), 1) * self.kmax * NUQ_BUCKET_GRAD_TILE,
+                                                 dtype=torch.float32, device=self.device))
+            _, gsegs, partial = self._grad_tables
+            _lib.check(self.L.pf_nuq_bucket_cluster_grad(_p(gsegs), _p(self.work_bg_dev), len(self.work_bg),
+                                                         _p(self.tiles_bg_dev), len(self.tiles_bg), self.kmax,
+                                                         _p(self.idx), _p(self.idx_base), _p(self.uq.scales),
+                                                         _p(partial), _p(grad_base), _p(self.cluster_off), _stream()),
+                       'pf_nuq_bucket_cluster_grad')
+            return
         if self._grad_tables is None or self._grad_tables[0] != ptrs:
             gs = self.uq.segs.copy()
             gs['src'] = ptrs
@@ -502,6 +621,11 @@ class CodebookWeightQuantizer:
                                               _p(first_dev), _p(self.idx), _p(self.idx_base), _p(self.uq.scales),
                                               _p(partial), _p(grad_base), _p(self.cluster_off), _stream()),
                    'pf_nuq_cluster_grad')
+
+    def bucket_storage_bits(self):
+        """Extra storage of the per-bucket alpha and beta, 64 bits per bucket (__updt_bucket_storage, utils.py:487-494);
+        the per-layer quantizer counts none."""
+        return self.uq.bucket_storage_bits() if self.use_buckets else 0
 
 
 # ----------------------------------------------------------------------------- a4 conv / a13 layers
